@@ -59,7 +59,19 @@ def parse():
     ap.add_argument("--cpu-sample-steps", type=int, default=60)
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--force-shard", action="store_true", help="shard the elimination tree even below SHARD_MIN_FLOPS")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (step direction, inertia) as DIR/<name>.npy, "
+                         "float64; the workload is seeded, so two builds run with the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+def dump_outputs(dirname, arrays):
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def load_workloads():
@@ -215,6 +227,8 @@ def run_reference(args, rank, world):
     model, st, its = make_workload(args.workload)
     la = _cpu_replay(st)
     dt, ms_fac = _cpu_run(la, its, args.warmup, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"direction": la.d.full(), "inertia": la.last_inertia})
     val = args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -343,12 +357,14 @@ def run_b200(args, rank, world, local_rank):
     pipe = HostIteratePipeline(la, FIELDS)
 
     def pipelined_steps(first, count):
-        """`count` host-facing steps; copies of neighbouring steps overlap the compute; returns device ms for all of them"""
+        """`count` host-facing steps; copies of neighbouring steps overlap the compute; returns device ms for all of them and
+        the index of the pinned host buffer that holds the last step's direction"""
         e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
         e0.record(stream)
         slot = pipe.prefetch(host[first % N_ITERATES])
         if not args.no_flush:
             flush_buf.fill_(1.0)                          # (inside the timed region here)
+        hs = None
         for j in range(count):
             i = first + j
             pipe.load(slot)
@@ -363,33 +379,38 @@ def run_b200(args, rank, world, local_rank):
             assert ok
             if not args.no_flush and j + 1 < count:
                 flush_buf.fill_(1.0)                      # L2 flush between steps, queued first so that it runs under the host's hand-over work
-            pipe.push_result()
+            hs = pipe.push_result()
             slot = nxt[0]
         pipe.drain()
         e1.record(stream)
         e1.synchronize()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), hs
 
     def timed_pipelined():
         pipelined_steps(0, args.warmup)
         barrier()
         t0 = time.perf_counter()
-        ms = pipelined_steps(args.warmup, args.steps)
+        ms, hs = pipelined_steps(args.warmup, args.steps)
         barrier()
         wall = time.perf_counter() - t0
         tot = torch.tensor([ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(tot, op=dist.ReduceOp.MAX)
-        return float(tot.item()), wall
+        return float(tot.item()), wall, hs
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
     dev_ms, dev_wall = timed_run(False)
     cnt_dev = dict(la.cnt)
+    if args.dump_outputs:
+        outputs = {"direction": la.d.values.cpu().numpy(), "inertia": la.last_inertia}
     ser_ms, ser_wall = timed_run(True)
-    e2e_ms, e2e_wall = timed_pipelined()
+    e2e_ms, e2e_wall, e2e_slot = timed_pipelined()
     assert pipe.h2d_bytes == h2d_bytes and pipe.d2h_bytes == d2h_bytes
+    if args.dump_outputs and rank == 0:
+        outputs["direction_e2e"] = pipe.d_host[e2e_slot].numpy()
+        dump_outputs(args.dump_outputs, outputs)
 
     # phase timings of the hot path's three metrics (SURVEY 8d M1/M2), measured separately from the step loop
     la.load_iterate(devit[0])

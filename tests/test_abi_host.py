@@ -193,3 +193,26 @@ def test_reference_arm_runs_without_the_product_library():
     class A: workload = "case300_synth"; no_flush = False
     class S: nvar = line["config"]["n"]; ncon = line["config"]["m"]
     assert line["config"] == bench.config_of(A, S, 1)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs DIR (reference arm): float64 .npy files of what the last of the --steps timed steps returned -- the same
+    on every run (seeded inputs) and equal to a replay of exactly --warmup + --steps steps; --steps 0 is refused."""
+    import subprocess, sys
+    import bench
+    cmd = [sys.executable, "bench.py", "--impl", "reference", "--steps", "3", "--warmup", "1", "--workload", "case300_synth"]
+    got = []
+    for name in ("a", "b"):
+        out = subprocess.run(cmd + ["--dump-outputs", str(tmp_path / name)], cwd=ROOT, capture_output=True, text=True, timeout=300)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert len([l for l in out.stdout.splitlines() if l.startswith("{")]) == 1
+        assert sorted(os.listdir(tmp_path / name)) == ["direction.npy", "inertia.npy"]
+        got.append({k: np.load(tmp_path / name / f"{k}.npy") for k in ("direction", "inertia")})
+    for k in ("direction", "inertia"):
+        assert got[0][k].dtype == np.float64 and np.array_equal(got[0][k], got[1][k]), k
+    model, st, its = bench.make_workload("case300_synth")
+    la = bench._cpu_replay(st)
+    bench._cpu_run(la, its, 1, 3)
+    assert np.array_equal(got[0]["direction"], la.d.full()) and tuple(got[0]["inertia"]) == tuple(la.last_inertia)
+    out = subprocess.run([sys.executable, "bench.py", "--steps", "0"], cwd=ROOT, capture_output=True, text=True, timeout=300)
+    assert out.returncode == 2 and "--steps" in out.stderr

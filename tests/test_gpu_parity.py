@@ -415,6 +415,27 @@ def test_host_pipeline_returns_the_same_directions_as_serial_steps():
         assert np.array_equal(a, b)
 
 
+def test_bench_dump_outputs_agree_with_the_reference_arm(tmp_path):
+    """bench.py --dump-outputs, both arms with the same arguments: the last timed step of the device-resident loop has the reference
+    arm's inertia and its step direction within 1e-6 (refined, as above); the pipelined host-facing loop returns it bit for bit."""
+    _need_gpu()
+    import os, subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    args = ["--steps", "3", "--warmup", "1", "--workload", "case300_synth", "--no-secondary", "--cpu-sample-steps", "0"]
+    got = {}
+    for impl in ("b200", "reference"):
+        out = subprocess.run([sys.executable, "bench.py", "--impl", impl, *args, "--dump-outputs", str(tmp_path / impl)],
+                             cwd=root, capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        got[impl] = {f[:-len(".npy")]: np.load(tmp_path / impl / f) for f in os.listdir(tmp_path / impl)}
+    g, r = got["b200"], got["reference"]
+    assert sorted(g) == ["direction", "direction_e2e", "inertia"] and sorted(r) == ["direction", "inertia"]
+    assert all(a.dtype == np.float64 for a in (*g.values(), *r.values()))
+    assert np.array_equal(g["inertia"], r["inertia"])
+    assert np.abs(g["direction"] - r["direction"]).max() / np.abs(r["direction"]).max() <= 1e-6
+    assert np.array_equal(g["direction_e2e"], g["direction"])
+
+
 def test_golden_fixture_on_device():
     """The committed HS15 fixture (tests/golden/hs15_kkt.json): factor + solve the stored condensed and augmented
     matrices through the C ABI and reproduce the stored solve_kkt vector / inertia."""
