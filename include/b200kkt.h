@@ -76,8 +76,19 @@ typedef struct b2_options {
                                 level of the critical path costs ~5 us of hand-off besides its pivots, the zeros nothing.
                                 Default 0 = off (measured slower on the OPF trees: the single-child chains sit at the bottom, where the
                                 tree is throughput-bound and bigger leaves hurt); kept as an option for trees with long chains on top */
-    int32_t reserved[4];
+    int32_t pivoting;        /* B2_PIVOT_*: pivoting of the dense solver (b2d_*).  The sparse solver (b2_*) supports only
+                                B2_PIVOT_STATIC and rejects any other value                                        */
+    int32_t reserved[3];
 } b2_options;
+
+#define B2_PIVOT_STATIC         0   /* 1 x 1 pivots in order, |d| < pivot_eps perturbed (default)                      */
+#define B2_PIVOT_BUNCH_KAUFMAN  1   /* dense solver: Bunch-Kaufman 1 x 1 / 2 x 2 pivots, search bounded to each 128 x 128
+                                       diagonal block; needs ceil(N / 128) <= number of SMs                              */
+/* pivot kinds reported by b2d_pivot_info */
+#define B2_PIVOT_KIND_1X1        0
+#define B2_PIVOT_KIND_2X2_FIRST  1
+#define B2_PIVOT_KIND_2X2_SECOND 2
+#define B2_PIVOT_KIND_PERTURBED  3  /* numerically zero column: pivot set to +-pivot_eps, counted as a zero eigenvalue */
 
 int b2_options_default(b2_options* opt);
 
@@ -175,14 +186,19 @@ int b2d_create(int32_t N, int32_t lda, const double* A_d, const b2_options* opt,
 int b2d_destroy(b2d_solver* s);
 /* Debug: device timeline of the dense look-ahead factorisation.  With B2_DENSE_TRACE=1 in the environment at b2d_create, every kernel
  * of b2d_factorize stamps %globaltimer (ns) at its first entry and last exit; slot = 8 * block column + kind (0 diagonal block, 1 near
- * trsm, 2 near syrk, 3 panel trsm, 4 block-column update, 5 trailing update, 6 inverse), two uint64 per slot.  *count = number of
- * uint64 values (0 when tracing is off); stamps are copied when capacity >= *count. */
+ * trsm, 2 near syrk, 3 panel trsm, 4 block-column update, 5 trailing update, 6 inverse, 7 Bunch-Kaufman diagonal block), two
+ * uint64 per slot.  *count = number of uint64 values (0 when tracing is off); stamps are copied when capacity >= *count. */
 int b2d_debug_trace(b2d_solver* s, uint64_t* stamps_h, int64_t capacity, int64_t* count);
 int b2d_factorize(b2d_solver* s, void* stream);
 int b2d_inertia(b2d_solver* s, int64_t* num_pos, int64_t* num_zero, int64_t* num_neg, void* stream);
 int b2d_inertia_enqueue(b2d_solver* s, void* stream);
 int b2d_inertia_fetch(b2d_solver* s, int64_t* num_pos, int64_t* num_zero, int64_t* num_neg);
 int b2d_solve(b2d_solver* s, double* x_d, int32_t nrhs, void* stream);
+/* Pivots of the last factorisation (host arrays of N entries; any pointer may be NULL); synchronises the device.
+ * perm_h[new] = old (the b2_get_perm convention): row `new` of P A P' is row `old` of A.  kind_h: B2_PIVOT_KIND_*.
+ * n_2x2: number of 2 x 2 pivots; n_perturbed: number of perturbed pivots.  A static-pivoting handle reports the identity,
+ * every kind 1 x 1 and n_2x2 = 0 (its perturbed pivots are counted in n_perturbed only). */
+int b2d_pivot_info(b2d_solver* s, int32_t* perm_h, int8_t* kind_h, int64_t* n_2x2, int64_t* n_perturbed);
 
 /* ------------------------------------------------------------------ assembly: COO -> CSC */
 /* Host, one-time: CSC pattern of a COO matrix with duplicate merging and the COO->CSC map

@@ -15,6 +15,8 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libb200kkt.so")
 B2_OK = 0
 B2_ERR_INVALID, B2_ERR_CUDA, B2_ERR_SYMBOLIC, B2_ERR_FACTORIZATION, B2_ERR_SOLVE, B2_ERR_NO_DEVICE = 1, 2, 3, 4, 5, 6
 ORDER_METIS_ND, ORDER_MINDEG, ORDER_NATURAL, ORDER_USER = 0, 1, 2, 3
+B2_PIVOT_STATIC, B2_PIVOT_BUNCH_KAUFMAN = 0, 1
+B2_PIVOT_KIND_1X1, B2_PIVOT_KIND_2X2_FIRST, B2_PIVOT_KIND_2X2_SECOND, B2_PIVOT_KIND_PERTURBED = 0, 1, 2, 3
 
 
 class B2Error(RuntimeError):
@@ -44,7 +46,8 @@ class Options(C.Structure):
     _fields_ = [
         ("ordering", C.c_int32), ("nemin", C.c_int32), ("relax_zeros", C.c_double), ("pivot_eps", C.c_double),
         ("use_cuda_graph", C.c_int32), ("small_front_max", C.c_int32), ("n_parts", C.c_int32), ("part_rank", C.c_int32),
-        ("kkt_n_primal", C.c_int32), ("fuse_max_fronts", C.c_int32), ("dep_schedule", C.c_int32), ("chain_merge_f", C.c_int32), ("reserved", C.c_int32 * 4),
+        ("kkt_n_primal", C.c_int32), ("fuse_max_fronts", C.c_int32), ("dep_schedule", C.c_int32), ("chain_merge_f", C.c_int32),
+        ("pivoting", C.c_int32), ("reserved", C.c_int32 * 3),
     ]
 
 
@@ -118,6 +121,7 @@ PROTOTYPES = {
     "b2d_inertia_enqueue": (C.c_int, [_p, _p]),
     "b2d_inertia_fetch": (C.c_int, [_p, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i64)]),
     "b2d_solve": (C.c_int, [_p, _p, _i32, _p]),
+    "b2d_pivot_info": (C.c_int, [_p, _p, _p, C.POINTER(_i64), C.POINTER(_i64)]),
     "b2_condensed_symbolic_device": (C.c_int, [_i32, _i32, _p, _p, _p, _p, _PP, C.POINTER(_i64), _p]),
     "b2_coo_to_csc_device": (C.c_int, [_i32, _i32, _i64, _p, _p, _p, _p, _p, C.POINTER(_i64), _p]),
     "b2d_ozaki_plan_create": (C.c_int, [_i32, _i32, _PP]),

@@ -10,7 +10,8 @@
 //   k_big_update_pipe (front_kernels.cuh)  trailing update with all 128 pivots at once.
 //
 // so a front of order N costs 3*N/128 dependent launches instead of 13*N/128, and the diagonal-block inversion is no
-// longer a separate pass.  Pivoting is static (front_kernels.cuh): |d| < eps is replaced by sign(d)*eps and counted.
+// longer a separate pass.  Pivoting is static (front_kernels.cuh): |d| < eps is replaced by sign(d)*eps and counted.  The dense
+// solver's opt-in Bunch-Kaufman mode replaces k_big_diag128 by k_bk_diag128 (bkpivot_kernels.cuh) and runs k_big_trsm<true>.
 #pragma once
 #include "front_kernels.cuh"
 
@@ -272,7 +273,11 @@ __global__ void __launch_bounds__(256, 1) k_big_diag128(FactorArgs a, const int3
 
 // L21 = A21 * Linv^T * D^{-1} for the rows below the diagonal block, in place.  GEMM view (transposed so that the
 // 128-wide side is the pivot-column index):  Ut(c, i) = sum_{k <= c} Linv(c, k) * A21(i, k);  tile 128 (c) x 64 (rows i).
+// PIV (Bunch-Kaufman, bkpivot_kernels.cuh): column c of the permuted A21 is column perm[kb + c] of the stored one, and each row
+// u = Ut(:, i) is rotated by the block's pair rotations before the division by Lambda:  L21' = A21 P' L11^{-T} Q_bd Lambda^{-1}.
+// In place is safe: a CTA has staged every column of its 64-row strip before its epilogue writes any of them.
 constexpr int TR_ROWS = GU_N;            // 64 rows of the front per CTA
+template <bool PIV>
 __global__ void __launch_bounds__(256, 2) k_big_trsm(FactorArgs a, const int32_t* __restrict__ list, int kb,
                                                      const double* __restrict__ Linv, const int64_t* __restrict__ linv_off, int bx0) {
     const int s = list[blockIdx.y];
@@ -310,7 +315,8 @@ __global__ void __launch_bounds__(256, 2) k_big_trsm(FactorArgs a, const int32_t
         for (int p = 0; p < GU_K / 4; ++p) {
             const int k = ch * GU_K + lb_k + 4 * p;
             const bool ok = b_ok && k < nb;
-            cp_async8_zfill(Bd + (lb_k + 4 * p) * GU_LDB, b_src + (size_t)(ok ? k : 0) * f, ok);
+            const int kc = PIV ? (ok ? a.perm[d.col0 + kb + k] - d.col0 - kb : 0) : (ok ? k : 0);
+            cp_async8_zfill(Bd + (lb_k + 4 * p) * GU_LDB, b_src + (size_t)kc * f, ok);
         }
     };
 #pragma unroll
@@ -360,7 +366,20 @@ __global__ void __launch_bounds__(256, 2) k_big_trsm(FactorArgs a, const int32_t
     __syncthreads();
     const int i = tid & (TR_ROWS - 1);
     if (r0 + i < f) {
-        for (int cc = tid >> 6; cc < nb; cc += 4) Lp[(size_t)(kb + cc) * f + r0 + i] = Cs[i * GU_LDC + cc] * dinv[cc];
+        for (int cc = tid >> 6; cc < nb; cc += 4) {
+            double u = Cs[i * GU_LDC + cc];
+            if (PIV) {                                                // (u Q)_c over a pair (p, p + 1), Q = [[cs, sn], [-sn, cs]]
+                const int kd = a.pkind[d.col0 + kb + cc];
+                if (kd == B2_PIVOT_KIND_2X2_FIRST) {
+                    const double cs = a.rot[d.col0 + kb + cc], sn = a.rot[d.col0 + kb + cc + 1];
+                    u = cs * u - sn * Cs[i * GU_LDC + cc + 1];
+                } else if (kd == B2_PIVOT_KIND_2X2_SECOND) {
+                    const double cs = a.rot[d.col0 + kb + cc - 1], sn = a.rot[d.col0 + kb + cc];
+                    u = sn * Cs[i * GU_LDC + cc - 1] + cs * u;
+                }
+            }
+            Lp[(size_t)(kb + cc) * f + r0 + i] = u * dinv[cc];
+        }
     }
     trace_exit(a, 8 * (kb / DB) + TR_TRSM);
 }

@@ -39,12 +39,17 @@ __device__ __forceinline__ double ds_poll(const double* p, int* err) {
 // vector it multiplies, so on the critical path (the newest y_c / x_c) the block is already there.  The CTA's own inverted
 // diagonal block sits in shared memory (cp.async at kernel start, padded rows: both the plain and the transposed apply are
 // bank-conflict free).
+// PIV: the factor of a Bunch-Kaufman factorisation (bkpivot_kernels.cuh), P A P' = L_bd Lambda L_bd' with L21' = L21 Q_bd.  Block k
+// loads b through perm, publishes y~_k = Q_k' y_k (what the stored L' multiplies), divides by Lambda, rotates the accumulated
+// z~_k - sum L'^T x_c by Q_k before Linv_k', and stores x through perm.  Everything stays inside the CTA that owns block k.
 constexpr int DS_LDI = BS + 1;
 constexpr size_t DS_SMEM = (size_t)(BS * DS_LDI + 2 * BS + 2 * 8 * BS + BS) * sizeof(double);
 
+template <bool PIV>
 __global__ void __launch_bounds__(DS_NT, 1) k_dense_solve_flow(int N, const double* __restrict__ L, const double* __restrict__ Linv,
                                                               const double* __restrict__ dvec, double* __restrict__ x,
-                                                              double* ybuf, double* xbuf, int* err) {
+                                                              double* ybuf, double* xbuf, int* err, const int32_t* __restrict__ perm,
+                                                              const int8_t* __restrict__ pkind, const double* __restrict__ rot) {
     extern __shared__ __align__(16) double ds_sm[];
     double* Ls = ds_sm;                                   // [BS][DS_LDI]: Ls[c*DS_LDI + r] = Linv_k(r, c)
     double (*vec)[BS] = (double (*)[BS])(Ls + BS * DS_LDI);                  // [2][BS] the block vector being applied
@@ -60,7 +65,8 @@ __global__ void __launch_bounds__(DS_NT, 1) k_dense_solve_flow(int N, const doub
         asm volatile("cp.async.commit_group;" ::: "memory");
     }
     // ---------------- forward
-    double t = (g == 0 && r < nb) ? x[kb + r] : 0.0;                         // group 0 carries the accumulator
+    const int xr = (PIV && r < nb) ? perm[kb + r] : kb + r;                  // row of x behind row kb + r of the (permuted) system
+    double t = (g == 0 && r < nb) ? x[xr] : 0.0;                             // group 0 carries the accumulator
     double v[16];
     for (int c = 0; c < k; ++c) {
         {                                                                     // L(kb + r, c*BS + g*16 + q), issued before the poll
@@ -98,8 +104,22 @@ __global__ void __launch_bounds__(DS_NT, 1) k_dense_solve_flow(int N, const doub
 #pragma unroll
         for (int u = 0; u < 8; ++u) yk += part[0][u][r];
         if (r >= nb) yk = 0.0;
-        ybuf[(size_t)k * BS + r] = yk;                                        // publish y_k (consumers: the block rows below)
     }
+    // pair rotation of block k at row r: kd = B2_PIVOT_KIND_*, (cs, sn) of its pair
+    int kd = B2_PIVOT_KIND_1X1;
+    double cs = 1.0, sn = 0.0;
+    if (PIV) {
+        if (g == 0 && r < nb) {
+            kd = pkind[kb + r];
+            if (kd == B2_PIVOT_KIND_2X2_FIRST) { cs = rot[kb + r]; sn = rot[kb + r + 1]; }
+            else if (kd == B2_PIVOT_KIND_2X2_SECOND) { cs = rot[kb + r - 1]; sn = rot[kb + r]; }
+            tk[r] = yk;
+        }
+        __syncthreads();
+        if (kd == B2_PIVOT_KIND_2X2_FIRST) yk = cs * yk - sn * tk[r + 1];         // y~ = Q' y
+        else if (kd == B2_PIVOT_KIND_2X2_SECOND) yk = sn * tk[r - 1] + cs * yk;
+    }
+    if (g == 0) ybuf[(size_t)k * BS + r] = yk;                                // publish y_k (consumers: the block rows below)
     // ---------------- diagonal + backward
     // s_k(j) -= sum_i L(cb + i, kb + j) x_c(i): a warp owns 4 columns j, its lanes stride the rows i (each load instruction reads
     // 32 consecutive rows of one column: coalesced), column sums meet through shuffles; `sacc` lives in the threads tid < BS
@@ -132,10 +152,21 @@ __global__ void __launch_bounds__(DS_NT, 1) k_dense_solve_flow(int N, const doub
     __syncthreads();
     if (g == 0) tk[r] = s;
     __syncthreads();
+    const double* sv = tk;
+    if (PIV) {                                                                // s = Q s~  (vec is free: the last poll has been consumed)
+        if (g == 0) {
+            double sr = s;
+            if (kd == B2_PIVOT_KIND_2X2_FIRST) sr = cs * s + sn * tk[r + 1];
+            else if (kd == B2_PIVOT_KIND_2X2_SECOND) sr = cs * s - sn * tk[r - 1];
+            vec[0][r] = sr;
+        }
+        __syncthreads();
+        sv = vec[0];
+    }
     {                                                                         // x_k = Linv_k' s_k : sum_{i >= r} Linv(i, r) s_i
         double acc = 0.0;
 #pragma unroll
-        for (int q = 0; q < 16; ++q) { const int i = g * 16 + q; acc = fma((i >= r) ? Ls[r * DS_LDI + i] : 0.0, tk[i], acc); }
+        for (int q = 0; q < 16; ++q) { const int i = g * 16 + q; acc = fma((i >= r) ? Ls[r * DS_LDI + i] : 0.0, sv[i], acc); }
         part[1][g][r] = acc;
     }
     __syncthreads();
@@ -145,7 +176,7 @@ __global__ void __launch_bounds__(DS_NT, 1) k_dense_solve_flow(int N, const doub
         for (int u = 0; u < 8; ++u) xk += part[1][u][r];
         if (r >= nb) xk = 0.0;
         xbuf[(size_t)k * BS + r] = xk;                                        // publish x_k (consumers: the block columns before)
-        if (r < nb) x[kb + r] = xk;
+        if (r < nb) x[xr] = xk;
     }
 }
 

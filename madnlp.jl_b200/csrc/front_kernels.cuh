@@ -40,10 +40,15 @@ struct FactorArgs {
     double eps;
     unsigned long long* trace = nullptr;   // debug (B2_DENSE_TRACE): [slot][2] = first entry / last exit of a launch, %globaltimer ns
     unsigned long long* ftrace = nullptr;  // debug (B2_SPARSE_TRACE): [supernode][3] = team starts / children assembled / front finished
+    // Bunch-Kaufman pivoting of the dense solver (bkpivot_kernels.cuh); all nullptr = static pivoting.  Per pivot (front order):
+    // perm[kb + i] = row of A that became row kb + i (global index), pkind = B2_PIVOT_KIND_*, rot = (cos, sin) over a 2 x 2 pair
+    int32_t* perm = nullptr;
+    int8_t* pkind = nullptr;
+    double* rot = nullptr;
 };
 
 // Timeline stamps of the dense look-ahead schedule (b2d_debug_trace): slot = 8 * block column + kernel kind
-enum { TR_DIAG = 0, TR_NEAR1 = 1, TR_NEAR2 = 2, TR_TRSM = 3, TR_COL = 4, TR_BULK = 5, TR_INV = 6 };
+enum { TR_DIAG = 0, TR_NEAR1 = 1, TR_NEAR2 = 2, TR_TRSM = 3, TR_COL = 4, TR_BULK = 5, TR_INV = 6, TR_BK = 7 };
 __device__ __forceinline__ unsigned long long global_ns() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
 __device__ __forceinline__ void trace_enter(const FactorArgs& a, int slot) {
     if (a.trace && threadIdx.x == 0) atomicMin(a.trace + 2 * slot, global_ns());

@@ -12,6 +12,7 @@
 #include "common.cuh"
 #include "front_kernels.cuh"
 #include "bigfactor_kernels.cuh"
+#include "bkpivot_kernels.cuh"
 #include "solve_kernels.cuh"
 #include "warp_kernels.cuh"
 #include "bigsolve_kernels.cuh"
@@ -109,20 +110,26 @@ inline bool lookahead_bulk() {
     static const bool on = [] { const char* e = getenv("B2_UPDATE_BULK"); return !e || atoi(e) != 0; }();
     return on;
 }
+// (a.perm set: Bunch-Kaufman diagonal block and the pivoted trsm; the trailing update is the same)
 void launch_big_step(const FactorArgs& a, const int32_t* lb, int nfronts, int ob, int maxf, double* Linv, const int64_t* linv_off,
                      cudaStream_t st, int64_t* nl) {
     static bool attr = false;
     if (!attr) {
         cudaFuncSetAttribute(k_big_diag128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Diag128Smem));
-        cudaFuncSetAttribute(k_big_trsm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
+        cudaFuncSetAttribute(k_bk_diag128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BkSmem));
+        cudaFuncSetAttribute(k_big_trsm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
+        cudaFuncSetAttribute(k_big_trsm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
         cudaFuncSetAttribute(k_big_update_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
         attr = true;
     }
-    k_big_diag128<<<nfronts, 256, sizeof(Diag128Smem), st>>>(a, lb, ob, Linv, linv_off, 1);
+    const bool piv = a.perm != nullptr;
+    if (piv) k_bk_diag128<<<nfronts, 256, sizeof(BkSmem), st>>>(a, lb, ob, Linv, linv_off);
+    else k_big_diag128<<<nfronts, 256, sizeof(Diag128Smem), st>>>(a, lb, ob, Linv, linv_off, 1);
     if (nl) ++*nl;
     const int rem = maxf - ob - 1;                  // rows below the first pivot of the block (upper bound over the fronts)
     if (rem <= 0) return;
-    k_big_trsm<<<dim3((rem + TR_ROWS - 1) / TR_ROWS, nfronts), 256, GU_SMEM, st>>>(a, lb, ob, Linv, linv_off, 0);
+    if (piv) k_big_trsm<true><<<dim3((rem + TR_ROWS - 1) / TR_ROWS, nfronts), 256, GU_SMEM, st>>>(a, lb, ob, Linv, linv_off, 0);
+    else k_big_trsm<false><<<dim3((rem + TR_ROWS - 1) / TR_ROWS, nfronts), 256, GU_SMEM, st>>>(a, lb, ob, Linv, linv_off, 0);
     if (lookahead_bulk()) {
         static bool battr = false;
         if (!battr) { cudaFuncSetAttribute(k_big_update_pipe_bulk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM_BULK); battr = true; }
@@ -192,7 +199,9 @@ void lookahead_attrs() {
     static bool attr = false;
     if (attr) return;
     cudaFuncSetAttribute(k_big_diag128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Diag128Smem));
-    cudaFuncSetAttribute(k_big_trsm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
+    cudaFuncSetAttribute(k_big_trsm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
+    cudaFuncSetAttribute(k_big_trsm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
+    cudaFuncSetAttribute(k_bk_diag128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BkSmem));
     cudaFuncSetAttribute(k_big_update_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
     cudaFuncSetAttribute(k_big_update_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
     cudaFuncSetAttribute(k_big_update_dyn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GU_SMEM);
@@ -206,6 +215,8 @@ void lookahead_attrs() {
 }
 
 // `list1`: device pointer to the front's supernode id; f, w: its order and pivot count.  Returns the number of launches.
+// a.perm set (Bunch-Kaufman pivoting of the dense solver): the general path throughout, with the pivoted diagonal block and trsm --
+// the near-diagonal kernels have no pivoted variant.
 int64_t enqueue_front_lookahead(const FactorArgs& a, const int32_t* list1, int f, int w, double* Linv, const int64_t* linv_off,
                                 LookaheadCtx& cx, cudaStream_t S1) {
     const LookaheadKnobs& K = lookahead_knobs();
@@ -221,14 +232,16 @@ int64_t enqueue_front_lookahead(const FactorArgs& a, const int32_t* list1, int f
     cudaEvent_t ev_bulk = nullptr, ev_side = nullptr;            // most recent R(.) / side-branch completion
     cudaEvent_t ev_bulk_prev = nullptr;                          // R(.) before the most recent one (depth-2 look-ahead)
     const int cw = K.depth2 ? 2 * DB : DB;                       // columns the side branch updates per panel
+    const bool piv = a.perm != nullptr;
     for (int k = 0; k < nb; ++k) {
         const int ob = k * DB;
         const int nbk = std::min(DB, w - ob);                    // pivots of this block column
         const int j1 = ob + nbk;                                 // first trailing row / column
         const int rem2 = f - (ob + 2 * DB);                      // rows / columns from the block after the next on
-        const bool near_step = K.use_near && ob + 2 * DB <= w;   // the next diagonal block is a full pivot block
+        const bool near_step = K.use_near && !piv && ob + 2 * DB <= w;   // the next diagonal block is a full pivot block
         const int with_inv = (near_step && K.inv_side) ? 0 : 1;  // inverse of this block formed on the side branch?
-        if (K.use_near && k > 0) launch_chain(k_big_diag128, dim3(1), sizeof(Diag128Smem), a, list1, ob, Linv, linv_off, with_inv);
+        if (piv) { k_bk_diag128<<<1, 256, sizeof(BkSmem), S1>>>(a, list1, ob, Linv, linv_off); ++nl; }
+        else if (K.use_near && k > 0) launch_chain(k_big_diag128, dim3(1), sizeof(Diag128Smem), a, list1, ob, Linv, linv_off, with_inv);
         else { k_big_diag128<<<1, 256, sizeof(Diag128Smem), S1>>>(a, list1, ob, Linv, linv_off, with_inv); ++nl; }
         if (j1 >= f) continue;                                   // no rows below (last block of a dense matrix)
         if (near_step) {
@@ -251,7 +264,7 @@ int64_t enqueue_front_lookahead(const FactorArgs& a, const int32_t* list1, int f
             }
             if (rem2 > 0) {
                 if (!K.inv_side) cudaStreamWaitEvent(S3, ev_diag, 0);
-                k_big_trsm<<<dim3((rem2 + TR_ROWS - 1) / TR_ROWS, 1), 256, GU_SMEM, S3>>>(a, list1, ob, Linv, linv_off, DB / TR_ROWS);
+                k_big_trsm<false><<<dim3((rem2 + TR_ROWS - 1) / TR_ROWS, 1), 256, GU_SMEM, S3>>>(a, list1, ob, Linv, linv_off, DB / TR_ROWS);
                 cudaEvent_t ev_panel = nullptr;
                 if (K.relax) { ev_panel = cx.ev(); cudaEventRecord(ev_panel, S3); }    // "panel k's L is complete"
                 cudaStreamWaitEvent(S3, ev_near, 0);
@@ -277,7 +290,8 @@ int64_t enqueue_front_lookahead(const FactorArgs& a, const int32_t* list1, int f
         }
         // general path: whole-panel trsm and the update of the next 128 columns on the chain, the rest on the bulk branch
         if (ev_side) cudaStreamWaitEvent(S1, ev_side, 0);
-        k_big_trsm<<<dim3((f - j1 + TR_ROWS - 1) / TR_ROWS, 1), 256, GU_SMEM, S1>>>(a, list1, ob, Linv, linv_off, 0);
+        if (piv) k_big_trsm<true><<<dim3((f - j1 + TR_ROWS - 1) / TR_ROWS, 1), 256, GU_SMEM, S1>>>(a, list1, ob, Linv, linv_off, 0);
+        else k_big_trsm<false><<<dim3((f - j1 + TR_ROWS - 1) / TR_ROWS, 1), 256, GU_SMEM, S1>>>(a, list1, ob, Linv, linv_off, 0);
         if (ev_bulk) cudaStreamWaitEvent(S1, ev_bulk, 0);                              // R(k-1) also wrote block column k+1
         const int jhi = std::min(f, ob + 2 * DB);
         k_big_update_pipe<<<dim3((f - j1 + GU_M - 1) / GU_M, (jhi - j1 + GU_N - 1) / GU_N, 1), 256, GU_SMEM, S1>>>(a, list1, ob, DB, DB, 2 * DB, 1);
@@ -806,6 +820,7 @@ int create_common(int32_t n, int64_t nnz, const int32_t* colptr_h, const int32_t
                   const b2_options* opt, const int32_t* user_perm_h, bool symbolic_only, b2_solver** out) {
     if (!out || !colptr_h || !rowval_h || n <= 0) { set_error("b2_create: invalid argument"); return B2_ERR_INVALID; }
     if (colptr_h[n] != nnz) { set_error("b2_create: colptr[n] != nnz"); return B2_ERR_INVALID; }
+    if (opt && opt->pivoting != B2_PIVOT_STATIC) { set_error("b2_create: pivoting mode not supported by the sparse solver"); return B2_ERR_INVALID; }
     b2_solver* s = new b2_solver();
     if (opt) s->opt = *opt; else b2_options_default(&s->opt);
     s->symbolic_only = symbolic_only;
@@ -1315,6 +1330,9 @@ struct b2d_solver {
     DevBuf<int64_t> linv_off;
     DevBuf<FrontDesc> desc;
     DevBuf<int32_t> list, counters;
+    DevBuf<int32_t> perm;                            // Bunch-Kaufman pivoting only: FactorArgs::perm / pkind / rot
+    DevBuf<int8_t> pkind;
+    DevBuf<double> rot;
     int32_t* h_counters = nullptr;
     cudaGraphExec_t g_factor = nullptr;
     cudaStream_t cap_stream = nullptr;
@@ -1336,10 +1354,16 @@ __global__ void k_copy_lower(int N, int lda, const double* __restrict__ A, doubl
         F[(size_t)j * N + i] = A[(size_t)j * lda + i];
 }
 
-void enqueue_dense_factor_lookahead(b2d_solver* s, cudaStream_t S1) {
+FactorArgs dense_factor_args(b2d_solver* s) {
     FactorArgs a;
     a.desc = s->desc.p; a.child_idx = nullptr; a.rel = nullptr; a.amap_src = nullptr; a.amap_dst = nullptr;
     a.A = nullptr; a.L = s->fact.p; a.ws = nullptr; a.dvec = s->dvec.p; a.counters = s->counters.p; a.eps = s->opt.pivot_eps;
+    a.perm = s->perm.p; a.pkind = s->pkind.p; a.rot = s->rot.p;       // (nullptr unless pivoting)
+    return a;
+}
+
+void enqueue_dense_factor_lookahead(b2d_solver* s, cudaStream_t S1) {
+    FactorArgs a = dense_factor_args(s);
     const int N = s->N, nb = (N + DB - 1) / DB;
     if (s->trace.p) {
         a.trace = s->trace.p;
@@ -1356,14 +1380,16 @@ void enqueue_dense_factor_lookahead(b2d_solver* s, cudaStream_t S1) {
 void enqueue_dense_factor(b2d_solver* s, cudaStream_t st) {
     static int lookahead = -1;
     if (lookahead < 0) { const char* e = getenv("B2_DENSE_LOOKAHEAD"); lookahead = e ? (atoi(e) != 0) : 1; }
-    if (lookahead && s->aux_stream && s->side_stream && s->N > 4 * DB) { enqueue_dense_factor_lookahead(s, st); return; }
-    FactorArgs a;
-    a.desc = s->desc.p; a.child_idx = nullptr; a.rel = nullptr; a.amap_src = nullptr; a.amap_dst = nullptr;
-    a.A = nullptr; a.L = s->fact.p; a.ws = nullptr; a.dvec = s->dvec.p; a.counters = s->counters.p; a.eps = s->opt.pivot_eps;
     const int N = s->N;
-    cudaMemsetAsync(s->counters.p, 0, 2 * sizeof(int32_t), st);     // [2] = sticky error flag of the dataflow solve
-    k_copy_lower<<<dim3(std::max(1, std::min(8, (N + 255) / 256)), N), 256, 0, st>>>(N, s->lda, s->A_d, s->fact.p);
-    for (int ob = 0; ob < N; ob += DB) launch_big_step(a, s->list.p, 1, ob, N, s->linv.p, s->linv_off.p, st, nullptr);
+    if (lookahead && s->aux_stream && s->side_stream && N > 4 * DB) enqueue_dense_factor_lookahead(s, st);
+    else {
+        FactorArgs a = dense_factor_args(s);
+        cudaMemsetAsync(s->counters.p, 0, 2 * sizeof(int32_t), st);     // [2] = sticky error flag of the dataflow solve
+        k_copy_lower<<<dim3(std::max(1, std::min(8, (N + 255) / 256)), N), 256, 0, st>>>(N, s->lda, s->A_d, s->fact.p);
+        for (int ob = 0; ob < N; ob += DB) launch_big_step(a, s->list.p, 1, ob, N, s->linv.p, s->linv_off.p, st, nullptr);
+    }
+    // Bunch-Kaufman: every block's interchanges reach the rows of the finished columns left of it
+    if (s->perm.p && N > DB) k_bk_swap_left<<<dim3(((N - 1) / DB) * DB, (N - 1) / DB), DB, 0, st>>>(N, s->fact.p, s->perm.p);
 }
 }  // namespace
 
@@ -1377,9 +1403,17 @@ int b2d_create(int32_t N, int32_t lda, const double* A_d, const b2_options* opt,
         set_error("b2d_create: no CUDA device (this library has no CPU fallback)");
         return B2_ERR_NO_DEVICE;
     }
+    b2_options o;
+    if (opt) o = *opt; else b2_options_default(&o);
+    if (o.pivoting != B2_PIVOT_STATIC && o.pivoting != B2_PIVOT_BUNCH_KAUFMAN) { set_error("b2d_create: unknown pivoting mode"); return B2_ERR_INVALID; }
+    // the pivoted solve is the single-launch dataflow kernel only: one resident CTA per 128-row block
+    if (o.pivoting == B2_PIVOT_BUNCH_KAUFMAN && (N + DB - 1) / DB > sm_count()) {
+        set_error("b2d_create: Bunch-Kaufman pivoting needs N <= 128 * (number of SMs) = " + std::to_string(DB * sm_count()));
+        return B2_ERR_INVALID;
+    }
     auto* s = new b2d_solver();
     s->N = N; s->lda = lda; s->A_d = A_d;
-    if (opt) s->opt = *opt; else b2_options_default(&s->opt);
+    s->opt = o;
     FrontDesc d;
     std::memset(&d, 0, sizeof(d));
     d.col0 = 0; d.w = N; d.f = N;
@@ -1395,7 +1429,9 @@ int b2d_create(int32_t N, int32_t lda, const double* A_d, const b2_options* opt,
         cudaStreamCreateWithFlags(&s->side_stream, cudaStreamNonBlocking) != cudaSuccess ||
         s->tilecnt.alloc((size_t)((N + DB - 1) / DB)) != cudaSuccess ||
         (getenv("B2_DENSE_TRACE") && atoi(getenv("B2_DENSE_TRACE")) && s->trace.alloc((size_t)16 * ((N + DB - 1) / DB)) != cudaSuccess) ||
-        cudaMemset(s->fact.p, 0, s->fact.bytes()) != cudaSuccess || cudaMemset(s->counters.p, 0, 4 * sizeof(int32_t)) != cudaSuccess) {
+        cudaMemset(s->fact.p, 0, s->fact.bytes()) != cudaSuccess || cudaMemset(s->counters.p, 0, 4 * sizeof(int32_t)) != cudaSuccess ||
+        (o.pivoting == B2_PIVOT_BUNCH_KAUFMAN &&
+         (s->perm.alloc(N) != cudaSuccess || s->pkind.alloc(N) != cudaSuccess || s->rot.alloc(N) != cudaSuccess))) {
         delete s;
         return cuda_fail(cudaGetLastError(), "b2d_create allocation", __FILE__, __LINE__);
     }
@@ -1469,16 +1505,26 @@ int b2d_solve(b2d_solver* s, double* x_d, int32_t nrhs, void* stream) {
     const int nblk = (N + BS - 1) / BS;
     static int flow_ok = -1;            // every CTA of the dataflow kernel must be resident: one per SM
     if (flow_ok < 0) {
-        flow_ok = cudaFuncSetAttribute(k_dense_solve_flow, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DS_SMEM) == cudaSuccess ? 1 : 0;
+        flow_ok = (cudaFuncSetAttribute(k_dense_solve_flow<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DS_SMEM) == cudaSuccess &&
+                   cudaFuncSetAttribute(k_dense_solve_flow<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DS_SMEM) == cudaSuccess) ? 1 : 0;
         if (const char* e = getenv("B2_DENSE_SOLVE_FLOW")) flow_ok = flow_ok && atoi(e) != 0;
+    }
+    const bool piv = s->perm.p != nullptr;
+    if (piv && !(flow_ok && nblk <= sm_count())) {
+        set_error("b2d_solve: the Bunch-Kaufman factor is solved by the single-launch kernel only, which is unavailable");
+        return B2_ERR_SOLVE;
     }
     for (int c = 0; c < nrhs; ++c) {
         double* x = x_d + (size_t)c * N;
         if (flow_ok && nblk <= sm_count()) {
             // ONE launch: block row / block column k is owned by CTA k, hand-off through sentinel-initialised vectors
             B2_CUDA(cudaMemsetAsync(s->flow.p, 0xFF, s->flow.bytes(), st));
-            k_dense_solve_flow<<<nblk, DS_NT, DS_SMEM, st>>>(N, s->fact.p, s->linv.p, s->dvec.p, x, s->flow.p, s->flow.p + (size_t)nblk * BS,
-                                                            s->counters.p + 2);
+            if (piv)
+                k_dense_solve_flow<true><<<nblk, DS_NT, DS_SMEM, st>>>(N, s->fact.p, s->linv.p, s->dvec.p, x, s->flow.p, s->flow.p + (size_t)nblk * BS,
+                                                                      s->counters.p + 2, s->perm.p, s->pkind.p, s->rot.p);
+            else
+                k_dense_solve_flow<false><<<nblk, DS_NT, DS_SMEM, st>>>(N, s->fact.p, s->linv.p, s->dvec.p, x, s->flow.p, s->flow.p + (size_t)nblk * BS,
+                                                                       s->counters.p + 2, nullptr, nullptr, nullptr);
             continue;
         }
         BigSolveArgs bs;
@@ -1497,6 +1543,29 @@ int b2d_solve(b2d_solver* s, double* x_d, int32_t nrhs, void* stream) {
         k_bs_bwd_finish<<<dim3((N + 255) / 256, 1), 256, 0, st>>>(bs, s->list.p);
     }
     B2_CUDA(cudaGetLastError());
+    return B2_OK;
+}
+
+int b2d_pivot_info(b2d_solver* s, int32_t* perm_h, int8_t* kind_h, int64_t* n_2x2, int64_t* n_perturbed) {
+    if (!s) { set_error("b2d_pivot_info: invalid argument"); return B2_ERR_INVALID; }
+    if (!s->factorized) { set_error("b2d_pivot_info: not factorized"); return B2_ERR_FACTORIZATION; }
+    B2_CUDA(cudaDeviceSynchronize());
+    const int N = s->N;
+    std::vector<int8_t> kind(N, (int8_t)B2_PIVOT_KIND_1X1);
+    int64_t n2 = 0, np = 0;
+    if (s->perm.p) {
+        B2_CUDA(cudaMemcpy(kind.data(), s->pkind.p, N * sizeof(int8_t), cudaMemcpyDeviceToHost));
+        if (perm_h) B2_CUDA(cudaMemcpy(perm_h, s->perm.p, N * sizeof(int32_t), cudaMemcpyDeviceToHost));
+        for (int8_t k : kind) { n2 += k == B2_PIVOT_KIND_2X2_FIRST; np += k == B2_PIVOT_KIND_PERTURBED; }
+    } else {
+        int32_t c[2];
+        B2_CUDA(cudaMemcpy(c, s->counters.p, sizeof(c), cudaMemcpyDeviceToHost));
+        np = c[1];
+        if (perm_h) for (int i = 0; i < N; ++i) perm_h[i] = i;
+    }
+    if (kind_h) std::memcpy(kind_h, kind.data(), N);
+    if (n_2x2) *n_2x2 = n2;
+    if (n_perturbed) *n_perturbed = np;
     return B2_OK;
 }
 

@@ -33,15 +33,20 @@ Base.@kwdef mutable struct B200Options <: AbstractOptions
     b200_fuse_max_fronts::Int32 = 8
     b200_dep_schedule::Int32 = 1
     b200_chain_merge_f::Int32 = 0
+    # B200DenseSolver only: MadNLP.BUNCHKAUFMAN (what LapackCPUSolver / LapackCUDASolver default to) selects Bunch-Kaufman
+    # pivoting (B2_PIVOT_BUNCH_KAUFMAN); `nothing` keeps the static 1 x 1 pivots.  The sparse solver always pivots statically.
+    lapack_algorithm::Union{Nothing,MadNLP.LinearFactorization} = nothing
 end
 
 struct CB2Options
     ordering::Int32; nemin::Int32; relax_zeros::Float64; pivot_eps::Float64
     use_cuda_graph::Int32; small_front_max::Int32; n_parts::Int32; part_rank::Int32
-    kkt_n_primal::Int32; fuse_max_fronts::Int32; dep_schedule::Int32; chain_merge_f::Int32; reserved::NTuple{4,Int32}
+    kkt_n_primal::Int32; fuse_max_fronts::Int32; dep_schedule::Int32; chain_merge_f::Int32
+    pivoting::Int32; reserved::NTuple{3,Int32}
 end
-CB2Options(o::B200Options) = CB2Options(o.b200_ordering, o.b200_nemin, o.b200_relax_zeros, o.b200_pivot_eps,
-    o.b200_use_cuda_graph, o.b200_small_front_max, 1, 0, o.b200_kkt_n_primal, o.b200_fuse_max_fronts, o.b200_dep_schedule, o.b200_chain_merge_f, ntuple(_ -> Int32(0), 4))
+CB2Options(o::B200Options; dense::Bool = false) = CB2Options(o.b200_ordering, o.b200_nemin, o.b200_relax_zeros, o.b200_pivot_eps,
+    o.b200_use_cuda_graph, o.b200_small_front_max, 1, 0, o.b200_kkt_n_primal, o.b200_fuse_max_fronts, o.b200_dep_schedule, o.b200_chain_merge_f,
+    Int32(dense && o.lapack_algorithm == MadNLP.BUNCHKAUFMAN ? 1 : 0), ntuple(_ -> Int32(0), 3))
 
 last_error() = unsafe_string(ccall((:b2_last_error, libb200kkt), Cstring, ()))
 function check(rc::Cint, exc)
@@ -217,7 +222,7 @@ end
 function B200DenseSolver(A::CuMatrix{Float64}; opt = B200Options(), logger = MadNLPLogger())
     N = size(A, 1); h = Ref{Ptr{Cvoid}}(C_NULL)
     check(ccall((:b2d_create, libb200kkt), Cint, (Int32, Int32, CuPtr{Float64}, Ptr{CB2Options}, Ptr{Ptr{Cvoid}}),
-        N, stride(A, 2), pointer(A), Ref(CB2Options(opt)), h), SymbolicException)
+        N, stride(A, 2), pointer(A), Ref(CB2Options(opt; dense = true)), h), SymbolicException)
     M = B200DenseSolver{Float64}(h[], A, C_NULL, C_NULL, opt, logger)
     finalizer(m -> ccall((:b2d_destroy, libb200kkt), Cint, (Ptr{Cvoid},), m.handle), M)
     return M
@@ -232,7 +237,8 @@ function inertia(M::B200DenseSolver)
     return (Int(p[]), Int(z[]), Int(n[]))
 end
 improve!(::B200DenseSolver) = false
-introduce(::B200DenseSolver) = "b200kkt dense LDL' (DMMA)"
+introduce(M::B200DenseSolver) =
+    M.opt.lapack_algorithm == MadNLP.BUNCHKAUFMAN ? "b200kkt dense LDL' (DMMA, Bunch-Kaufman pivoting)" : "b200kkt dense LDL' (DMMA, static pivoting)"
 input_type(::Type{<:B200DenseSolver}) = :dense
 default_options(::Type{<:B200DenseSolver}) = B200Options()
 is_supported(::Type{<:B200DenseSolver}, ::Type{Float64}) = true

@@ -120,8 +120,13 @@ class B200SparseSolver:
 class B200DenseSolver:
     """Blocked dense LDL^T on the fp64 tensor pipe (role of LapackCUDASolver / LapackCPUSolver{BUNCHKAUFMAN},
     src/LinearSolvers/lapack.jl:164-172, cusolver.jl:150-187).  `A` is an N x N column-major device matrix kept by
-    reference; only its lower triangle is read."""
+    reference; only its lower triangle is read.
+
+    Pivoting: ``default_options(pivoting="static")`` (default) takes 1 x 1 pivots in order and perturbs |d| < pivot_eps;
+    ``pivoting="bunchkaufman"`` takes Bunch-Kaufman 1 x 1 / 2 x 2 pivots with the search bounded to each 128 x 128 diagonal
+    block (N <= 128 * number of SMs)."""
     input_type = "dense"
+    PIVOTING = {"static": capi.B2_PIVOT_STATIC, "bunchkaufman": capi.B2_PIVOT_BUNCH_KAUFMAN}
 
     def __init__(self, A, opt: capi.Options | None = None, stream=None):
         capi.require_device()
@@ -140,8 +145,12 @@ class B200DenseSolver:
             lib.b2d_destroy(h)
             self._h = None
 
-    @staticmethod
-    def default_options(**kw):
+    @classmethod
+    def default_options(cls, **kw):
+        if isinstance(kw.get("pivoting"), str):
+            if kw["pivoting"] not in cls.PIVOTING:
+                raise ValueError(f"pivoting must be one of {sorted(cls.PIVOTING)}, not {kw['pivoting']!r}")
+            kw["pivoting"] = cls.PIVOTING[kw["pivoting"]]
         return capi.default_options(**kw)
 
     @staticmethod
@@ -149,7 +158,17 @@ class B200DenseSolver:
         return np.dtype(dtype) == np.float64
 
     def introduce(self) -> str:
-        return f"b200kkt dense LDL^T (DMMA) v{lib.b2_version()}"
+        mode = "Bunch-Kaufman pivoting" if self.opt.pivoting == capi.B2_PIVOT_BUNCH_KAUFMAN else "static pivoting"
+        return f"b200kkt dense LDL^T (DMMA, {mode}) v{lib.b2_version()}"
+
+    def pivot_info(self):
+        """pivots of the last factorisation: (perm, kind, n_2x2, n_perturbed) with perm[new] = old and kind[i] one of
+        capi.B2_PIVOT_KIND_*; a static-pivoting solver reports the identity and only 1 x 1 pivots"""
+        perm = np.empty(self.n, dtype=np.int32)
+        kind = np.empty(self.n, dtype=np.int8)
+        n2, npert = C.c_int64(), C.c_int64()
+        check(lib.b2d_pivot_info(self._h, perm.ctypes.data, kind.ctypes.data, C.byref(n2), C.byref(npert)))
+        return perm, kind, n2.value, npert.value
 
     def is_async(self) -> bool:
         return True
